@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA path through the C-ABI)
   python bench.py --impl reference --gpus N --steps K ...   the reference's CPU path (cv2) on host cores
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's results to DIR/<name>.npy
 
 A "step" is one pass of the hot path over one batch of synthetic 1920x1080 frames (16 markers of
 DICT_6X6_250 each): BGR8 frames -> ids, corners, rvec/tvec, quaternion, image/object error, area,
@@ -408,6 +409,32 @@ def parity_gate(frames, idx, out, dict_id, K, D, maxm):
             "bars": "ids identical and in identical order; corners, tvec, quaternion <= 1e-3 vs oracle/aruco_oracle.py (cv2) on frames of the timed batch"}
 
 
+def map_rows(entries):
+    """fid_map_entry list -> float64 rows: fiducial_id, num_obs, x, y, z, rx, ry, rz, variance."""
+    return np.array([[e.fiducial_id, e.num_obs, e.x, e.y, e.z, e.rx, e.ry, e.rz, e.variance] for e in entries], np.float64).reshape(-1, 9)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array, so that two builds can be compared output for output on identical inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
+
+
+def detection_arrays(out, maxm):
+    """The results of one batch as a caller of the detect/pose path receives them, without the unused slots past each frame's
+    count: markers in frame order, then in the order the library reports them."""
+    from fiducials_b200.node import FiducialSlam
+
+    counts, ids, corners, tfs = out
+    nf = len(counts)
+    valid = np.arange(maxm)[None, :] < counts[:, None]
+    tf = np.frombuffer(bytes(tfs), FiducialSlam.TRANSFORM_DTYPE).reshape(nf, maxm)[valid]
+    return {"counts": counts, "ids": ids[valid], "corners": corners.reshape(nf, maxm, 4, 2)[valid], "translation": tf["translation"], "rotation": tf["rotation"],
+            "rvec": tf["rvec"], "image_error": tf["image_error"], "object_error": tf["object_error"], "fiducial_area": tf["fiducial_area"]}
+
+
 # ------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------
@@ -522,6 +549,8 @@ def run_gpu_arm(args):
     stage_ms = det.last_stage_ms()  # stages of the last batch call (nf frames)
     counters = det.last_counters()
     last_out = outs[(args.steps - 1) & 3]
+    if args.dump_outputs and rank == 0:  # before the e2e pass reuses the output buffers
+        dump_outputs(args.dump_outputs, dict(detection_arrays(last_out, MAXM), map_entries=map_rows(slam.entries()), merged_map_entries=map_rows(slam.merged_entries())))
     e2e_s, e2e_wall, _, _ = timed(False, args.steps)
     clocks = sampler.stop()
     n_merged = len(slam.merged_entries())
@@ -728,6 +757,8 @@ def run_c5(args, reference):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     dt = float(t[0])
     ents = slam.entries(0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"map_entries": map_rows(ents)})
     # the north-star's batched SE(3) Gauss-Newton over the same observations (fid_map_refine; new, parity unpinned): cost, the
     # reference's plane-fit metric (fiducial_slam/scripts/fit_plane.py; the synthetic ceiling is the plane z = 2.5) and wall time
     refine = None
@@ -781,11 +812,16 @@ def run_c5(args, reference):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C2", choices=["C2", "C3", "C4", "C5"], help="BASELINE.json config (the driver's default, C2, is the one the metric is quoted on)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32/float64; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     global WORKLOAD
     WORKLOAD = args.workload
     claim_stdout()

@@ -2,8 +2,9 @@
 unmodified from /root/reference against the stand-in headers of oracle/ref_shim; built by oracle/Makefile where the reference
 checkout exists, shipped prebuilt to the GPU box).
 
-TEST INFRASTRUCTURE ONLY -- never imported by the product (fiducials_b200/).  It pins oracle/slam_oracle.py (tests/test_map_ref.py)
-and checks the CUDA map update (tests/test_gpu_slam.py) against the reference code itself rather than against a restatement."""
+TEST INFRASTRUCTURE ONLY -- never imported by the product (fiducials_b200/).  tests/golden/make_map_ref_golden.py records its answers
+into tests/golden/map_ref_golden.npz, against which tests/test_map_ref.py pins oracle/slam_oracle.py and tests/test_gpu_slam.py
+checks the CUDA map update: the reference code itself rather than a restatement, without needing the reference checkout."""
 import ctypes as C
 import os
 import tempfile
